@@ -50,6 +50,8 @@ def parse():
     ap.add_argument("--voc-pair-kmax", type=int, default=None, help="override hifigan.Generator.pair_kmax (largest kernel size run as fused pairs)")
     ap.add_argument("--voc-pair-mask", type=int, default=None, help="override hifigan.Generator.pair_mask (A/B of the per-pair fused launches)")
     ap.add_argument("--fs2-f8", type=int, default=None, choices=[0, 1], help="override the decoder / PostNet operand split (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (rank 0) as DIR/<name>.npy, to compare two builds output for output")
     return ap.parse_args()
 
 
@@ -158,6 +160,26 @@ class ClockSampler:
         busy = [c for c, w in zip(sm, pw) if w > 250.0] or sm          # samples taken under load (idle draw is ~150 W)
         return {"sm_mhz": statistics.median(busy), "sm_mhz_min": min(busy), "sm_mhz_last_samples": busy[-4:], "sm_max_mhz": max(mx), "power_w_max": max(pw), "samples": len(sm), "samples_under_load": len(busy),
                 "reasons": sorted(reasons), "sampler": self.mode, "query_ms_max": max(qms) if qms else None}
+
+
+OUTPUT_NAMES = ("mel", "postnet_mel", "p_pred", "e_pred", "log_d_pred", "d_rounded", "src_masks", "mel_masks", "src_lens", "mel_lens")
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """Write each array as `directory/<name>.npy`: floating point as float32, integers and masks as float64 (exact).  If they come to
+    more than 64 MB in all, every array above 1 MB is cut to the same fraction of its elements, taken evenly spaced over the flattened
+    array, so that runs with the same arguments sample the same positions."""
+    import numpy as np
+    arrays = {k: v.astype(np.float32 if np.issubdtype(v.dtype, np.floating) else np.float64) for k, v in arrays.items()}
+    big = {k for k, a in arrays.items() if a.nbytes > 1 << 20}
+    room = DUMP_BYTES - 4096 * len(arrays) - sum(a.nbytes for k, a in arrays.items() if k not in big)     # (4 KB per .npy header)
+    keep = min(1.0, room / max(1, sum(arrays[k].nbytes for k in big)))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        if name in big and keep < 1.0:
+            a = a.reshape(-1)[np.linspace(0, a.size - 1, int(a.size * keep)).astype(np.int64)]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def workload_config(args, world, frames_per_utt):
@@ -409,9 +431,14 @@ def run_ours(args):
     del out, wav                                      # (timed() keeps at most one previous result set alive, like the warm-up loop)
 
     # N > 1: the asynchronous gather of the last step completes inside the timed region (flush before the closing event)
-    ms_total, launches, _ = timed(step_device, args.steps) if gather is None else _timed_with_flush(timed, step_device, gather, args.steps, args.prime)
+    ms_total, launches, last = timed(step_device, args.steps) if gather is None else _timed_with_flush(timed, step_device, gather, args.steps, args.prime)
     clocks = sampler.stop() if sampler else None
     spread_device = dict(timed.spread)
+    if args.dump_outputs and rank == 0:
+        out, wav = last
+        dump_outputs(args.dump_outputs, {**{n: t.cpu().numpy() for n, t in zip(OUTPUT_NAMES, out)}, "wav": wav.cpu().numpy()})
+        del out, wav
+    del last
     value = samples_step * args.steps / (ms_total * 1e-3)
 
     ms_mel, _, _ = timed(lambda: model(spk, texts, lens, L), args.steps)

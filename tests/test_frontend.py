@@ -131,53 +131,51 @@ def test_device_batches_on_cuda_stage_through_pinned_slots(tmp_path):
         assert torch.equal(s_t, torch.from_numpy(spk)) and torch.equal(t_t, torch.from_numpy(texts)) and torch.equal(l_t, torch.from_numpy(lens))
 
 
-def test_against_the_reference_dataloader_on_its_shipped_val_files():
-    """The three `preprocessed_data/*/val.txt` files the reference ships (512 utterances each, English ARPAbet and Mandarin pinyin),
-    through the reference's own TextDataset + DataLoader(batch_size=8) + to_device, against TextBatches / device_batches and against
-    OUR TextDataset under the same stock DataLoader.  Runs in a subprocess: the reference's module names (`text`, `utils`, `dataset`)
-    must resolve to its tree."""
-    from oracle import ref_import
-    if not ref_import.available():
-        pytest.skip("reference tree not present")
-    code = r'''
-import sys, os
-sys.path.insert(0, %r)
-from oracle import ref_import
-ref_import._stub()
-REF = ref_import.REFERENCE_ROOT
-sys.path.insert(0, REF); os.chdir(REF)
-import numpy as np, torch, yaml
-from torch.utils.data import DataLoader
-from dataset import TextDataset as RefTextDataset
-from utils.tools import to_device
-from text import text_to_sequence
-from fastspeech2_b200 import frontend
-n = 0
-for ds_name in ("LJSpeech", "LibriTTS", "AISHELL3"):
-    pc = yaml.safe_load(open(f"config/{ds_name}/preprocess.yaml"))
-    src = os.path.join(pc["path"]["preprocessed_path"], "val.txt")
-    ref = RefTextDataset(src, pc)
-    want = list(DataLoader(ref, batch_size=8, collate_fn=ref.collate_fn))
-    ours_ds = frontend.TextDataset(src, pc)                      # default text_to_sequence: the tree's own `text` package
-    via_loader = list(DataLoader(ours_ds, batch_size=8, collate_fn=ours_ds.collate_fn))
-    tb = frontend.TextBatches(src, pc, batch_size=8, text_to_sequence=text_to_sequence)
-    direct, dev = list(tb), list(tb.device_batches("cpu"))
-    assert len(want) == len(via_loader) == len(direct) == len(dev) == 64
-    for w, a, b, d in zip(want, via_loader, direct, dev):
-        for got in (a, b):
-            assert got[0] == w[0] and got[1] == w[1] and got[5] == w[5] and type(got[5]) is type(w[5])
+def test_against_the_reference_dataloader_on_its_shipped_val_files(tmp_path):
+    """Every 8th line of the three `preprocessed_data/*/val.txt` files the reference ships (English ARPAbet and Mandarin pinyin):
+    TextBatches / device_batches and OUR TextDataset under a stock DataLoader(batch_size=8), against the batches the reference's own
+    TextDataset + DataLoader produced (tests/golden/frontend_val.npz, oracle/gen_golden.py gen_frontend).  Phoneme ids are the
+    reference's text_to_sequence output, recorded per utterance."""
+    import torch
+    from torch.utils.data import DataLoader
+    z = np.load(os.path.join(ROOT, "tests", "golden", "frontend_val.npz"))
+    n = 0
+    for ds_name in ("LJSpeech", "LibriTTS", "AISHELL3"):
+        g = lambda k: z[f"{ds_name}_{k}"]
+        lines, cleaners = [str(l) for l in g("lines")], json.loads(str(g("cleaners")))
+        phones = np.split(g("phones"), np.cumsum(g("phone_lens"))[:-1])
+        seq_of = {l.split("|")[2]: p for l, p in zip(lines, phones)}
+
+        def t2s(text, c):
+            assert c == cleaners
+            return seq_of[text]
+
+        d = tmp_path / ds_name
+        d.mkdir()
+        (d / "val.txt").write_text("\n".join(lines) + "\n", encoding="utf-8")
+        (d / "speakers.json").write_text(str(g("speaker_map")))
+        src, pc = str(d / "val.txt"), {"preprocessing": {"text": {"text_cleaners": cleaners}}, "path": {"preprocessed_path": str(d)}}
+        sizes, mxs = g("batch_sizes"), g("max_len")
+        rows, flat = np.cumsum(np.r_[0, sizes]), np.cumsum(np.r_[0, sizes * mxs])
+        want = [(list(g("ids")[rows[b]:rows[b + 1]]), list(g("raw")[rows[b]:rows[b + 1]]), g("speakers")[rows[b]:rows[b + 1]],
+                 g("texts")[flat[b]:flat[b + 1]].reshape(sizes[b], mxs[b]), g("text_lens")[rows[b]:rows[b + 1]], mxs[b]) for b in range(len(sizes))]
+        ours_ds = frontend.TextDataset(src, pc, text_to_sequence=t2s)
+        via_loader = list(DataLoader(ours_ds, batch_size=8, collate_fn=ours_ds.collate_fn))
+        tb = frontend.TextBatches(src, pc, batch_size=8, text_to_sequence=t2s)
+        direct, dev = list(tb), list(tb.device_batches("cpu"))
+        assert len(want) == len(via_loader) == len(direct) == len(dev) == 8
+        for w, a, b, dv in zip(want, via_loader, direct, dev):
+            for got in (a, b):
+                assert got[0] == w[0] and got[1] == w[1] and got[5] == w[5] and type(got[5]) is type(w[5])
+                for i in (2, 3, 4):
+                    assert got[i].dtype == w[i].dtype and got[i].shape == w[i].shape and np.array_equal(got[i], w[i]), (ds_name, i)
+            assert dv[0] == w[0] and dv[1] == w[1] and dv[5] == w[5]
             for i in (2, 3, 4):
-                assert got[i].dtype == w[i].dtype and got[i].shape == w[i].shape and np.array_equal(got[i], w[i]), (ds_name, i)
-        wd = to_device(w, torch.device("cpu"))
-        assert d[0] == wd[0] and d[1] == wd[1] and d[5] == wd[5]
-        for i in (2, 3, 4):
-            assert d[i].dtype == wd[i].dtype and torch.equal(d[i], wd[i])
-        n += len(w[0])
-    item_r, item_o = ref[5], ours_ds[5]
-    assert item_r[0] == item_o[0] and item_r[1] == item_o[1] and np.array_equal(item_r[2], item_o[2]) and item_r[3] == item_o[3]
-    print(ds_name, "padding", round(tb.padded_fraction(), 3), "->", round(frontend.TextBatches(src, pc, batch_size=8, bucket=True, text_to_sequence=text_to_sequence).padded_fraction(), 3))
-print("compared", n)
-''' % ROOT
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "compared 1536" in r.stdout, r.stdout + r.stderr
-    print(r.stdout)
+                assert dv[i].dtype == torch.int64 and torch.equal(dv[i], torch.from_numpy(w[i]).long())
+            n += len(w[0])
+        speaker_map = json.loads(str(g("speaker_map")))
+        for i, line in enumerate(lines):
+            name, spk, _, raw = line.split("|")
+            item = ours_ds[i]
+            assert item[0] == name and item[1] == speaker_map[spk] and np.array_equal(item[2], phones[i]) and item[3] == raw
+    assert n == 192

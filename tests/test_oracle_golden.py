@@ -2,7 +2,7 @@
 
 tests/golden/*.npz were produced by the UNMODIFIED reference (oracle/gen_golden.py); the oracle must reproduce them.
 fp32 oracle vs reference: same ATen kernels -> bit-identical at one thread; a few ulp otherwise (thread-count dependent
-reduction order, SURVEY.md Appendix D).  When the reference tree is present the comparison is also run live."""
+reduction order, SURVEY.md Appendix D)."""
 import json
 import os
 
@@ -12,7 +12,7 @@ import torch
 
 from fastspeech2_b200 import configs, synth
 from oracle import fs2_oracle as O
-from oracle import ref_import
+from oracle.gen_golden import golden_sample
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -106,59 +106,45 @@ def test_remove_weight_norm_matches_oracle_fold():
         assert torch.allclose(v, folded[k], rtol=1e-6, atol=1e-8), k
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not present (GPU box)")
+def _assert_pinned(z, prefix, out, tol=5e-6):
+    for i in range(5):
+        assert tuple(out[i].shape) == tuple(z[f"{prefix}{i}_shape"]), (prefix, i)
+        assert np.abs(golden_sample(out[i].numpy()) - z[f"{prefix}{i}"]).max() < tol, (prefix, i)
+
+
 def test_oracle_vs_live_reference(scratch):
-    FastSpeech2, hifigan = ref_import.load()
+    """LibriTTS with pitch / duration control, the teacher-forced path on the reference's own predictions, and a second
+    random-weight Generator: oracle vs the outputs the unmodified reference recorded (oracle/gen_golden.py gen_pins)."""
+    z = np.load(os.path.join(GOLD, "oracle_pins_libri.npz"))
     pc, mc = configs.make_configs("LibriTTS", scratch)
-    sd = synth.fastspeech2_state_dict(pc, mc, seed=31)
-    ref = FastSpeech2(pc, mc)
-    ref.load_state_dict(sd)
-    ref.eval()
-    spk, texts, lens, L = synth.make_batch(3, 36, seed=32, n_speakers=904, min_len=10)
-    with torch.no_grad():
-        want = ref(spk, texts, lens, L, p_control=0.9, d_control=1.2)
+    sd = synth.fastspeech2_state_dict(pc, mc, seed=int(z["seed"]))
+    t = lambda k: torch.from_numpy(z[k])
+    spk, texts, lens, L = t("speakers"), t("texts"), t("src_lens"), int(z["max_src_len"])
     got = O.fastspeech2_forward(sd, spk, texts, lens, L, p_control=0.9, d_control=1.2)
-    assert torch.equal(got[9], want[9]) and torch.equal(got[5], want[5])
-    for i in range(5):
-        assert (got[i] - want[i]).abs().max() < 5e-6
+    assert torch.equal(got[9], t("mel_lens")) and torch.equal(got[5], t("d_rounded"))
+    _assert_pinned(z, "out", got)
     # teacher-forced path
-    d_t, ml = want[5].long(), want[9]
-    with torch.no_grad():
-        want2 = ref(spk, texts, lens, L, None, ml, int(ml.max()), want[2], want[3], d_t)
-    got2 = O.fastspeech2_forward(sd, spk, texts, lens, L, None, ml, int(ml.max()), want[2], want[3], d_t)
-    for i in range(5):
-        assert (got2[i] - want2[i]).abs().max() < 5e-6
-    h = hifigan.AttrDict(configs.HIFIGAN_CONFIG)
-    hsd = synth.hifigan_state_dict(h, seed=33)
-    gen = hifigan.Generator(h)
-    gen.load_state_dict(hsd)
-    gen.eval()
-    gen.remove_weight_norm()
-    mel = synth.make_mel(1, 30, seed=34)
-    with torch.no_grad():
-        w = gen(mel)
-    assert (O.hifigan_forward(hsd, mel) - w).abs().max() < 1e-5
+    ml = t("mel_lens")
+    got2 = O.fastspeech2_forward(sd, spk, texts, lens, L, None, ml, int(ml.max()), t("p_pred"), t("e_pred"), t("d_rounded").long())
+    _assert_pinned(z, "teacher", got2)
+    hsd = synth.hifigan_state_dict(configs.HIFIGAN_CONFIG, seed=int(z["hifigan_seed"]))
+    wav = O.hifigan_forward(hsd, t("hifigan_mel"))
+    assert tuple(wav.shape) == tuple(z["wav_shape"])
+    assert np.abs(golden_sample(wav.numpy()) - z["wav"]).max() < 1e-5
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not present (GPU box)")
 def test_oracle_frame_level_vs_live_reference(scratch):
-    """frame_level pitch / energy (config/LJSpeech_paper, model/modules.py:139-148): oracle vs the unmodified reference."""
+    """frame_level pitch / energy (config/LJSpeech_paper, model/modules.py:139-148): oracle vs the outputs the unmodified reference
+    recorded (oracle/gen_golden.py gen_pins)."""
     import copy
-    FastSpeech2, _ = ref_import.load()
+    z = np.load(os.path.join(GOLD, "oracle_pins_frame_level.npz"))
     pc, mc = configs.make_configs("LJSpeech", scratch)
     pc = copy.deepcopy(pc)
     pc["preprocessing"]["pitch"]["feature"] = "frame_level"
     pc["preprocessing"]["energy"]["feature"] = "frame_level"
-    sd = synth.fastspeech2_state_dict(pc, mc, seed=41)
-    ref = FastSpeech2(pc, mc)
-    ref.load_state_dict(sd)
-    ref.eval()
-    spk, texts, lens, L = synth.make_batch(2, 22, seed=42, min_len=13)
-    with torch.no_grad():
-        want = ref(spk, texts, lens, L, p_control=1.2)
-    got = O.fastspeech2_forward(sd, spk, texts, lens, L, p_control=1.2, pitch_level="frame_level", energy_level="frame_level")
-    assert torch.equal(got[9], want[9]) and got[2].shape == want[2].shape == want[0].shape[:2]
-    for i in range(5):
-        assert (got[i] - want[i]).abs().max() < 5e-6
+    sd = synth.fastspeech2_state_dict(pc, mc, seed=int(z["seed"]))
+    t = lambda k: torch.from_numpy(z[k])
+    got = O.fastspeech2_forward(sd, t("speakers"), t("texts"), t("src_lens"), int(z["max_src_len"]), p_control=float(z["p_control"]),
+                                pitch_level="frame_level", energy_level="frame_level")
+    assert torch.equal(got[9], t("mel_lens")) and torch.equal(got[5], t("d_rounded")) and got[2].shape == got[0].shape[:2]
+    _assert_pinned(z, "out", got)
