@@ -223,7 +223,8 @@ __global__ void durations_kernel(const fs2_durations_args a) {
       if (a.use_target) {
         d = s;
       } else {
-        d = fmaxf(rintf(expf(s) - 1.f) * a.d_control, 0.f);
+        d = rintf(expf(s) - 1.f) * a.d_control;
+        d = isnan(d) ? d : fmaxf(d, 0.f);  // torch.clamp(min=0) keeps a NaN (fmaxf alone would turn it into 0 frames, uncounted)
         if (a.d_rounded) a.d_rounded[(long long)b * a.L + l] = d;
       }
       // int() truncation toward zero.  A NaN / inf / absurd duration (the reference raises on int(inf) or dies allocating) is counted
@@ -481,8 +482,16 @@ int transpose_bct_to_btc(const float* in, float* out, int B, int C, int T, cudaS
 }
 
 // ------------------------------------------------------------------ waveform -> int16 + per-utterance trim (utils/model.py:82-90)
-// out[b][t] = t < lens[b] ? (int16) trunc(wav[b][t] * scale) : 0.  numpy's astype("int16") truncates toward zero; values beyond the
-// int16 range (|wav| >= 1 after tanh: not reachable) are clamped instead of wrapping.  One thread converts 8 samples (16-byte store).
+// out[b][t] = t < lens[b] ? np_int16(wav[b][t] * scale) : 0, where np_int16 is numpy's float32 -> int16 astype on x86-64: truncate
+// toward zero to int32 (cvttss2si), then keep the low 16 bits.  So the conversion wraps: wav == 1.0 -- which tanhf returns exactly for
+// arguments >= ~9.01 -- gives -32768, and NaN, +-inf and anything outside int32 give INT32_MIN, whose low 16 bits are 0.
+// One thread converts 8 samples (16-byte store).
+__device__ __forceinline__ short np_int16(float v) {
+  const float t = truncf(v);
+  if (!(t >= -2147483648.f && t < 2147483648.f)) return 0;
+  return (short)(int)t;  // modulo 2^16
+}
+
 __global__ void wav_to_int16_kernel(const float* __restrict__ wav, long long wav_bs, const long long* __restrict__ lens, float scale, int B,
                                     long long N, short* __restrict__ out) {
   const long long per_b = (N + 7) / 8;
@@ -497,10 +506,10 @@ __global__ void wav_to_int16_kernel(const float* __restrict__ wav, long long wav
     const float4 a = __ldg(reinterpret_cast<const float4*>(src)), c = __ldg(reinterpret_cast<const float4*>(src) + 1);
     const float f[8] = {a.x, a.y, a.z, a.w, c.x, c.y, c.z, c.w};
 #pragma unroll
-    for (int k = 0; k < 8; k++) v[k] = t0 + k < len ? (short)min(max(__float2int_rz(f[k] * scale), -32768), 32767) : (short)0;
+    for (int k = 0; k < 8; k++) v[k] = t0 + k < len ? np_int16(__fmul_rn(f[k], scale)) : (short)0;
   } else {
 #pragma unroll
-    for (int k = 0; k < 8; k++) v[k] = (t0 + k < N && t0 + k < len) ? (short)min(max(__float2int_rz(src[k] * scale), -32768), 32767) : (short)0;
+    for (int k = 0; k < 8; k++) v[k] = (t0 + k < N && t0 + k < len) ? np_int16(__fmul_rn(src[k], scale)) : (short)0;
   }
   short* dst = out + (long long)b * N + t0;
   if (t0 + 8 <= N && ((reinterpret_cast<uintptr_t>(dst) & 15u) == 0)) {

@@ -31,7 +31,8 @@ def vocoder_infer(mels, vocoder, model_config, preprocess_config, lengths=None):
     """Drop-in for the reference's `utils.model.vocoder_infer` (utils/model.py:74-92), same arguments and return value (a list of
     int16 numpy arrays, one per utterance, trimmed to `lengths[i]` samples).  The reference copies the fp32 waveform to the host
     and converts / trims there; here `x max_wav_value -> int16` and the trim run on the device (fs2_wav_to_int16), so 2 bytes per
-    sample cross PCIe, into pinned memory, asynchronously on the compute stream."""
+    sample cross PCIe, into pinned memory, asynchronously on the compute stream.  The conversion is numpy's: out-of-range samples wrap
+    (a waveform sample of exactly 1.0 becomes -32768) and NaN / inf become 0, so the int16 samples equal the reference's."""
     import torch
 
     from . import ops

@@ -39,12 +39,13 @@ def conv1d(x, w, bias=None, *, dilation=1, pad_left=0, in_act=L.ACT_NONE, in_slo
     return out
 
 
-def layernorm(x, gamma, beta, row_lens=None, eps=1e-5):
+def layernorm(x, gamma, beta, row_lens=None, eps=1e-5, pre_relu=False):
+    """LayerNorm over the last dim (of relu(x) with pre_relu), rows t >= row_lens[b] zeroed (fs2_layernorm)."""
     _need_cuda(x)
     B, T, Cc = x.shape
     y = torch.empty_like(x)
     a = L.LayerNormArgs(x=x.data_ptr(), y=y.data_ptr(), B=B, T=T, C=Cc, gamma=gamma.data_ptr(), beta=beta.data_ptr(), eps=eps,
-                        row_lens=L.ptr(row_lens))
+                        row_lens=L.ptr(row_lens), pre_relu=int(pre_relu))
     L.check(L.lib().fs2_layernorm(C.byref(a), _stream(x.device)), "fs2_layernorm")
     return y
 
@@ -148,7 +149,8 @@ def resstack(x, kernels, dilations, w1_tc, b1, w2_tc, b2, alpha=0.0, out=None, a
 
 
 def wav_to_int16(wav, lengths=None, scale=32768.0, out=None):
-    """wav [B,N] fp32 (row-strided ok) -> int16 [B,N]: trunc(wav*scale), samples t >= lengths[b] zeroed (fs2_wav_to_int16)."""
+    """wav [B,N] fp32 (row-strided ok) -> int16 [B,N]: numpy's (wav*scale).astype("int16") (truncates, wraps beyond int16), samples
+    t >= lengths[b] zeroed (fs2_wav_to_int16)."""
     _need_cuda(wav)
     B, N = wav.shape
     assert wav.stride(1) == 1

@@ -155,7 +155,8 @@ int fs2_variance_head(const fs2_variance_head_args* a, fs2_stream_t stream);
 
 /* d = use_target ? src[b,l] : max(rint(exp(src[b,l]) - 1) * d_control, 0); reps = max((int)d, 0);
  * cum[b,l] = inclusive prefix sum of reps; mel_lens[b] = cum[b,L-1]; len_stats[0] = max_b mel_lens, [1] = sum_b mel_lens,
- * [2] = number of non-finite / > 1e6 durations (those contribute 0 frames; the reference raises on them).  The call zeroes len_stats. */
+ * [2] = number of non-finite / > 1e6 durations (those contribute 0 frames; the reference raises on them).  The call zeroes len_stats.
+ * max() keeps a NaN, like torch.clamp(min=0): a NaN log-duration is written to d_rounded as NaN and counted in len_stats[2]. */
 typedef struct fs2_durations_args {
   const float* src; int use_target; float d_control; int B, L;
   float* d_rounded;     /* [B][L] or NULL */
@@ -202,7 +203,9 @@ int fs2_resstack_plan(const fs2_resstack_args* a, int num_sms, int32_t* out);
 
 /* out[b,t] = t < lens[b] ? (int16) trunc(wav[b,t] * scale) : 0   -- the device half of utils.model.vocoder_infer (utils/model.py:82-90:
  * `(wavs.cpu().numpy() * max_wav_value).astype("int16")` then `wavs[i][:lengths[i]]`): 2 bytes per sample cross PCIe instead of 4, the
- * trim is fused, and the copy can be asynchronous.  lens (samples, int64, device) may be NULL.  Values beyond int16 are clamped. */
+ * trim is fused, and the copy can be asynchronous.  lens (samples, int64, device) may be NULL; lens[b] < 0 keeps nothing, > N keeps all.
+ * Values beyond int16 wrap like the reference's numpy cast: trunc to int32, keep the low 16 bits (wav = 1.0 -> -32768); NaN, +-inf and
+ * values outside int32 give 0. */
 typedef struct fs2_wav_int16_args {
   const float* wav; int64_t wav_batch_stride; int B; int64_t N;
   const int64_t* lens; float scale; int16_t* out; /* [B][N] contiguous */
