@@ -13,7 +13,8 @@
 //
 // Roles: warp 0 streams K / V stages (cp.async.bulk), warp 1 issues the MMAs, warps 2-9 are "row" warps (TMEM lane quarter =
 // warp % 4, column half = (warp-2)/4): Q conversion, both softmax passes, the epilogue.
-#include "conv_tc_kernel.cuh"
+#include "common.cuh"
+#include "tc_format.cuh"
 
 namespace fs2 {
 
@@ -22,9 +23,6 @@ int pack_kv_tiles(const fs2_attention_args* a, unsigned char* kt, unsigned char*
 constexpr int AF_THREADS = 320;
 constexpr int AF_SB = 8;                         // K / V stage ring depth
 constexpr uint32_t AF_STAGE = 8192;              // one stage: [hi | lo][2 chunks][128][16 B]
-constexpr float AF_WSCALE = 16.f;                // operand scale of the packed K / V tiles (attention_tc.cu::AT_WSCALE)
-
-__device__ __forceinline__ void row_warps_sync_af() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 row warps only
 
 struct AfP {
   const float* qkv; float* ctx;
@@ -36,18 +34,14 @@ struct AfP {
 
 // 16 fp32 values of one row -> fp16 hi / lo operand planes of K-block kb ([2 chunks][128 rows][16 B] each)
 __device__ __forceinline__ void af_store16(unsigned char* kblk, int row, const float (&a)[16]) {
-  uint32_t hw[8], lw[8];
-#pragma unroll
-  for (int j = 0; j < 8; j++) {
-    hw[j] = cvt_f16x2_sat(a[2 * j], a[2 * j + 1]);
-    const float2 hf = __half22float2(*reinterpret_cast<const __half2*>(&hw[j]));
-    lw[j] = cvt_f16x2_sat(a[2 * j] - hf.x, a[2 * j + 1] - hf.y);
-  }
+  uint32_t hw[2][4], lw[2][4];
+  split_f16(a, hw[0], lw[0]);
+  split_f16(a + 8, hw[1], lw[1]);
   unsigned char* p0 = kblk + (size_t)row * 16;
-  *reinterpret_cast<uint4*>(p0) = make_uint4(hw[0], hw[1], hw[2], hw[3]);                 // hi, chunk 0
-  *reinterpret_cast<uint4*>(p0 + 2048) = make_uint4(hw[4], hw[5], hw[6], hw[7]);          // hi, chunk 1
-  *reinterpret_cast<uint4*>(p0 + 4096) = make_uint4(lw[0], lw[1], lw[2], lw[3]);          // lo, chunk 0
-  *reinterpret_cast<uint4*>(p0 + 6144) = make_uint4(lw[4], lw[5], lw[6], lw[7]);          // lo, chunk 1
+  *reinterpret_cast<uint4*>(p0) = make_uint4(hw[0][0], hw[0][1], hw[0][2], hw[0][3]);          // hi, chunk 0
+  *reinterpret_cast<uint4*>(p0 + 2048) = make_uint4(hw[1][0], hw[1][1], hw[1][2], hw[1][3]);   // hi, chunk 1
+  *reinterpret_cast<uint4*>(p0 + 4096) = make_uint4(lw[0][0], lw[0][1], lw[0][2], lw[0][3]);   // lo, chunk 0
+  *reinterpret_cast<uint4*>(p0 + 6144) = make_uint4(lw[1][0], lw[1][1], lw[1][2], lw[1][3]);   // lo, chunk 1
 }
 
 __global__ void __launch_bounds__(AF_THREADS, 1) attention_fused_kernel(const AfP p) {
@@ -74,12 +68,9 @@ __global__ void __launch_bounds__(AF_THREADS, 1) attention_fused_kernel(const Af
     for (int i = 0; i < AF_SB; i++) { mbar_init(&fullB[i], 1); mbar_init(&emptyB[i], 1); }
     for (int i = 0; i < 2; i++) { mbar_init(&sFull[i], 1); mbar_init(&sEmpty[i], 8); }
     mbar_init(qReady, 8); mbar_init(pReady, 8); mbar_init(pFree, 1); mbar_init(oFull, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, 512);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -113,8 +104,7 @@ __global__ void __launch_bounds__(AF_THREADS, 1) attention_fused_kernel(const Af
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    uint32_t leader;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(leader));
+    const uint32_t leader = elect_one();
     const uint32_t idesc = umma_idesc_f16(128);
     const uint64_t desc_c = umma_desc(0, 2048, 128);     // A and B alike: chunk stride 128 rows * 16 B, 8-row groups 128 B apart
     const uint32_t qa16 = smem_u32(qa) >> 4, pa16 = smem_u32(pa) >> 4;
@@ -167,7 +157,7 @@ __global__ void __launch_bounds__(AF_THREADS, 1) attention_fused_kernel(const Af
     const int r128 = q * 32 + lane;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
     const int D = p.H * 128;
-    const float c = p.scale * (1.f / AF_WSCALE) * 1.4426950408889634f;      // s*c = scaled score in log2 units (K tiles carry x16)
+    const float c = p.scale * (1.f / KV_WSCALE) * 1.4426950408889634f;      // s*c = scaled score in log2 units (K tiles carry x16)
     uint32_t s_phase[2] = {0, 0}, pf_phase = 0, o_phase = 0;
     bool p_written = false;
     for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
@@ -218,9 +208,9 @@ __global__ void __launch_bounds__(AF_THREADS, 1) attention_fused_kernel(const Af
         if (lane == 0) mbar_arrive(&sEmpty[sb]);
       }
       xch[h * 128 + r128] = m;
-      row_warps_sync_af();
+      row_warps_sync<256>();
       m = fmaxf(xch[r128], xch[128 + r128]);
-      row_warps_sync_af();                          // xch is reused for the row sums
+      row_warps_sync<256>();                          // xch is reused for the row sums
       // ---- pass 2: p = exp2(s*c - m) -> P operand planes (this warp: keys 64h .. 64h+63 of the block = K-blocks 4h .. 4h+3)
       float l = 0.f;
       for (int j = 0; j < nkb; j++) {
@@ -252,12 +242,12 @@ __global__ void __launch_bounds__(AF_THREADS, 1) attention_fused_kernel(const Af
         p_written = true;
       }
       xch[h * 128 + r128] = l;
-      row_warps_sync_af();
+      row_warps_sync<256>();
       l = xch[r128] + xch[128 + r128];
       // ---- epilogue: O / l (V tiles carry x16), rows beyond the utterance are zero
       mbar_wait(oFull, o_phase); o_phase ^= 1;
       tc_fence_after();
-      const float inv = (t < len) ? (1.f / AF_WSCALE) / l : 0.f;
+      const float inv = (t < len) ? (1.f / KV_WSCALE) / l : 0.f;
       float* dst = p.ctx + ((long long)b * p.T + t) * D + hd * 128 + h * 64;
 #pragma unroll
       for (int g = 0; g < 2; g++) {
@@ -270,7 +260,7 @@ __global__ void __launch_bounds__(AF_THREADS, 1) attention_fused_kernel(const Af
                                                                       __uint_as_float(ov[4 * k4 + 2]) * inv, __uint_as_float(ov[4 * k4 + 3]) * inv);
         }
       }
-      row_warps_sync_af();                          // xch free for the next item
+      row_warps_sync<256>();                          // xch free for the next item
     }
   }
 
@@ -278,17 +268,15 @@ __global__ void __launch_bounds__(AF_THREADS, 1) attention_fused_kernel(const Af
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
+    tmem_dealloc(tmem, 512);
   }
 }
 
 static constexpr size_t AF_SMEM = 2 * 65536 + (size_t)AF_SB * AF_STAGE + 256 * 4 + (2 * AF_SB + 10) * 8 + 16;
 
-static inline long long af_tile_stride(int Tk) { return TC_HDR + (long long)Tk * 512; }
-
 size_t attention_fused_workspace(int B, int T, int H) {
   const int Tk = (T + 127) / 128 * 128;
-  const size_t tile_bytes = ((size_t)B * H * af_tile_stride(Tk) + 255) & ~(size_t)255;
+  const size_t tile_bytes = ((size_t)B * H * kv_tile_stride(Tk) + 255) & ~(size_t)255;
   return 2 * tile_bytes + 256;
 }
 
@@ -300,17 +288,11 @@ int attention_fused(const fs2_attention_args* a, void* ws, size_t ws_bytes, cuda
   int derr = FS2_OK;
   DevState* dv = dev_state(&derr);
   if (!dv) return derr;
-  if (!dv->att_fused_ready.load(std::memory_order_acquire)) {
-    DevOnce once;
-    if (!dv->att_fused_ready.load(std::memory_order_relaxed)) {
-      cudaError_t e = cudaFuncSetAttribute(attention_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AF_SMEM);
-      if (e != cudaSuccess) return FS2_ERR_CUDA - (int)e;
-      dv->att_fused_ready.store(true, std::memory_order_release);
-    }
-  }
+  FS2_TRY(setup_once(dv->att_fused_ready,
+                     [] { return cudaFuncSetAttribute(attention_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AF_SMEM); }));
   const int Tk = (a->T + 127) / 128 * 128;
   char* base = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-  const long long tstride = af_tile_stride(Tk);
+  const long long tstride = kv_tile_stride(Tk);
   const size_t tile_bytes = ((size_t)a->B * a->H * tstride + 255) & ~(size_t)255;
   unsigned char* kt = reinterpret_cast<unsigned char*>(base);
   unsigned char* vt = kt + tile_bytes;

@@ -175,14 +175,8 @@ int attention_simt(const fs2_attention_args* a, cudaStream_t s) {
   int derr = FS2_OK;
   DevState* dv = dev_state(&derr);
   if (!dv) return derr;
-  if (!dv->att_simt_ready.load(std::memory_order_acquire)) {
-    DevOnce once;
-    if (!dv->att_simt_ready.load(std::memory_order_relaxed)) {
-      cudaError_t e = cudaFuncSetAttribute(attention_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ATT_SMEM);
-      if (e != cudaSuccess) return FS2_ERR_CUDA - (int)e;
-      dv->att_simt_ready.store(true, std::memory_order_release);
-    }
-  }
+  FS2_TRY(setup_once(dv->att_simt_ready,
+                     [] { return cudaFuncSetAttribute(attention_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ATT_SMEM); }));
   dim3 grid((a->T + ATT_BQ - 1) / ATT_BQ, a->H, a->B);
   prof_before(s);
   attention_simt_kernel<<<grid, 256, ATT_SMEM, s>>>(*a);

@@ -12,9 +12,8 @@
 //
 // The score matrix is materialised once in fp32 (the reference writes it four times); a fused flash-style tcgen05 kernel
 // that keeps S in TMEM is the planned replacement.  The exact fp32 kernel (attention_simt.cu) stays in use for the encoder.
-#include <cuda_fp16.h>
-
 #include "common.cuh"
+#include "tc_format.cuh"
 
 namespace fs2 {
 
@@ -22,9 +21,10 @@ int conv1d_tc(const fs2_conv1d_args* a, const float* wt, unsigned variant, cudaS
 
 constexpr int AT_DH = 128;          // head width
 constexpr int AT_NB = 128;          // output-channel block of the GEMM engine for N = 128*k
-constexpr int AT_HDR = 128;         // tile-buffer header bytes
-constexpr float AT_WSCALE = 16.f;   // power-of-two operand scale of the K / V tiles (|k|, |v| < 4094 stay inside fp16)
 
+// Not split_f16 (tc_format.cuh): this split scales, clamps with fminf / fmaxf and then rounds, so a NaN input becomes -65504 where
+// the saturating convert of split_f16 keeps the NaN.  Sharing the split would change what both attention backends return for
+// non-finite K / V.
 __device__ __forceinline__ void split8(const float (&f)[8], float scale, uint4& hi, uint4& lo) {
   uint32_t hw[4], lw[4];
 #pragma unroll
@@ -61,12 +61,12 @@ __device__ __forceinline__ void pack_k_tiles(const float* __restrict__ qkv, unsi
     f[0] = u.x; f[1] = u.y; f[2] = u.z; f[3] = u.w; f[4] = v.x; f[5] = v.y; f[6] = v.z; f[7] = v.w;
   }
   uint4 hi, lo;
-  split8(f, AT_WSCALE, hi, lo);
+  split8(f, KV_WSCALE, hi, lo);
   unsigned char* base = tiles + (long long)bh * tile_stride;
-  if (key == 0 && dchunk == 0) *reinterpret_cast<float*>(base) = 1.f / AT_WSCALE;
+  if (key == 0 && dchunk == 0) *reinterpret_cast<float*>(base) = 1.f / KV_WSCALE;
   const int nblk = key / AT_NB, nn = key - nblk * AT_NB, kb = dchunk >> 1, chunk = dchunk & 1;
   const size_t b_plane = 2 * AT_NB * 16, stage = 2 * b_plane, kbl = AT_DH / 16;
-  unsigned char* dst = base + AT_HDR + ((size_t)nblk * kbl + kb) * stage + ((size_t)chunk * AT_NB + nn) * 16;
+  unsigned char* dst = base + TC_HDR + ((size_t)nblk * kbl + kb) * stage + ((size_t)chunk * AT_NB + nn) * 16;
   *reinterpret_cast<uint4*>(dst) = hi;
   *reinterpret_cast<uint4*>(dst + b_plane) = lo;
 }
@@ -89,12 +89,12 @@ __device__ __forceinline__ void pack_v_tiles(const float* __restrict__ qkv, unsi
     f[e] = key < T ? __ldg(qkv + ((long long)b * T + key) * 3 * D + 2 * D + h * AT_DH + d) : 0.f;
   }
   uint4 hi, lo;
-  split8(f, AT_WSCALE, hi, lo);
+  split8(f, KV_WSCALE, hi, lo);
   unsigned char* base = tiles + (long long)bh * tile_stride;
-  if (k8 == 0 && d == 0) *reinterpret_cast<float*>(base) = 1.f / AT_WSCALE;
+  if (k8 == 0 && d == 0) *reinterpret_cast<float*>(base) = 1.f / KV_WSCALE;
   const int kb = k8 >> 1, chunk = k8 & 1;
   const size_t b_plane = 2 * AT_NB * 16, stage = 2 * b_plane;
-  unsigned char* dst = base + AT_HDR + (size_t)kb * stage + ((size_t)chunk * AT_NB + d) * 16;
+  unsigned char* dst = base + TC_HDR + (size_t)kb * stage + ((size_t)chunk * AT_NB + d) * 16;
   *reinterpret_cast<uint4*>(dst) = hi;
   *reinterpret_cast<uint4*>(dst + b_plane) = lo;
 }
@@ -154,8 +154,6 @@ __global__ void softmax_rows_kernel(float* __restrict__ S, int B, int T, int Tk,
   }
 }
 
-static inline long long at_tile_stride(int Tk) { return AT_HDR + (long long)Tk * 512; }   // 128 d x 2 planes x 2 bytes per key
-
 // K / V operand tiles of every (utterance, head) for the GEMM engine (also used by the fused kernel, attention_fused.cu)
 int pack_kv_tiles(const fs2_attention_args* a, unsigned char* kt, unsigned char* vt, long long tstride, cudaStream_t s) {
   const int B = a->B, T = a->T, H = a->H;
@@ -172,7 +170,7 @@ int pack_kv_tiles(const fs2_attention_args* a, unsigned char* kt, unsigned char*
 size_t attention_gemm_workspace(int B, int T, int H) {
   const int Tk = (T + 127) / 128 * 128;
   const size_t s_bytes = ((size_t)B * H * T * Tk * sizeof(float) + 255) & ~(size_t)255;
-  const size_t tile_bytes = ((size_t)B * H * at_tile_stride(Tk) + 255) & ~(size_t)255;
+  const size_t tile_bytes = ((size_t)B * H * kv_tile_stride(Tk) + 255) & ~(size_t)255;
   return s_bytes + 2 * tile_bytes + 256;
 }
 
@@ -186,7 +184,7 @@ int attention_gemm(const fs2_attention_args* a, void* ws, size_t ws_bytes, cudaS
   char* base = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
   float* S = reinterpret_cast<float*>(base);
   const size_t s_bytes = ((size_t)B * H * T * Tk * sizeof(float) + 255) & ~(size_t)255;
-  const long long tstride = at_tile_stride(Tk);
+  const long long tstride = kv_tile_stride(Tk);
   const size_t tile_bytes = ((size_t)B * H * tstride + 255) & ~(size_t)255;
   unsigned char* kt = reinterpret_cast<unsigned char*>(base + s_bytes);
   unsigned char* vt = kt + tile_bytes;

@@ -31,17 +31,16 @@ inline int cuda_status() {
 
 // Per-device one-time setup (SM count, >48 KB dynamic shared memory opt-ins).  cudaFuncSetAttribute applies to the CURRENT device's
 // context, so the "done" flags are kept per device ordinal; dev_state() looks the current device up (thread-safe) and
-// DevOnce serialises the first call per (device, kernel family).
+// setup_once() runs a kernel family's setup the first time the family is used on that device.
 constexpr int FS2_MAX_DEVICES = 64;
 struct DevState {
   std::atomic<int> num_sms{0};
   std::atomic<bool> conv_tc_ready{false}, att_simt_ready{false}, fused_ready{false}, att_fused_ready{false};
 };
 DevState* dev_state(int* err);                       // NULL + *err on failure
-struct DevOnce {                                     // RAII lock around a first-use setup section
-  DevOnce();
-  ~DevOnce();
-};
+// Runs fn unless `done` (a DevState flag) is set, and sets it once fn has succeeded; first calls from several threads are
+// serialised.  Returns FS2_OK or the CUDA error of fn.
+int setup_once(std::atomic<bool>& done, cudaError_t (*fn)());
 
 // optional per-launch event timing (see fs2_profile_begin in fs2b200.h); armed per host thread
 extern thread_local bool g_prof_on;

@@ -145,17 +145,13 @@ int conv1d_tc(const fs2_conv1d_args* a, const float* wt, unsigned variant, cudaS
   int derr = FS2_OK;
   DevState* dv = dev_state(&derr);                      // state of the CURRENT device: the caller's stream must belong to it
   if (!dv) return derr;
-  if (!dv->conv_tc_ready.load(std::memory_order_acquire)) {
-    DevOnce once;
-    if (!dv->conv_tc_ready.load(std::memory_order_relaxed)) {
-      const int mx = 227 * 1024;
-      cudaError_t e = conv_tc_prepare_mt1(mx);
-      if (e == cudaSuccess) e = conv_tc_prepare_mt2(mx);
-      if (e == cudaSuccess) e = conv_tc_prepare_mt4(mx);
-      if (e != cudaSuccess) return FS2_ERR_CUDA - (int)e;
-      dv->conv_tc_ready.store(true, std::memory_order_release);
-    }
-  }
+  FS2_TRY(setup_once(dv->conv_tc_ready, [] {
+    const int mx = 227 * 1024;
+    cudaError_t e = conv_tc_prepare_mt1(mx);
+    if (e == cudaSuccess) e = conv_tc_prepare_mt2(mx);
+    if (e == cudaSuccess) e = conv_tc_prepare_mt4(mx);
+    return e;
+  }));
   const int g_num_sms = dv->num_sms.load(std::memory_order_relaxed);
   TcP p{};
   p.x = a->x; p.xbs = a->x_batch_stride; p.xrs = a->x_row_stride;

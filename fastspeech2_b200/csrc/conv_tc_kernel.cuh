@@ -29,9 +29,8 @@
 //               row's 128 bytes -> bias / activation / residual / alpha / accumulate / pad-row mask -> full-line global I/O.
 //               Runs on work item i while the MMAs of item i+1 fill the other accumulator set.
 #pragma once
-#include <cuda_fp16.h>
-
 #include "common.cuh"
+#include "tc_format.cuh"
 
 namespace fs2 {
 
@@ -44,7 +43,6 @@ constexpr int TC_TTHREADS = TC_TW * 32;
 constexpr int TC_THREADS = 64 + TC_TTHREADS + 128;   // producer + MMA warps, transform warps, 4 epilogue warps
 constexpr int TC_DEPTH = 3;         // K-blocks of activation loads in flight per transform thread (register ring)
 constexpr int TC_LD = 3;           // (row, K-chunk) items (2 float4 loads each) per transform thread per K-block: 256 * 3 / 2 >= 384 rows
-constexpr int TC_HDR = 128;        // bytes of header in front of the weight tiles: float[0] = 1 / weight scale
 constexpr int TC_STAGE_FLOATS = 32 * 36;   // per-epilogue-warp transpose tile
 
 struct TcP {
@@ -82,123 +80,6 @@ struct TcP {
   int f8;                          // operand split: 0 = three kind::f16 MMAs (hi*hi + lo*hi + hi*lo), 1 = kind::f16 main term + ONE kind::f8f6f4 correction MMA
 };
 
-// ------------------------------------------------------------------ PTX wrappers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-// Programmatic dependent launch: the grid may start while its predecessor in the stream is still draining; everything that
-// reads or writes memory the predecessor touches comes after grid_dep_wait() (returns once the predecessor has completed and
-// flushed).  grid_dep_launch() lets the successor's CTAs be scheduled onto SMs as this grid's CTAs exit.
-__device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void grid_dep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tc_mma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// kind::f8f6f4 with E4M3 operands (K = 32 per instruction: here 16 channels x {activation-lo * weight-hi, activation-hi * weight-lo})
-__device__ __forceinline__ void tc_mma_f8(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
-        "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
-        "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// 8 consecutive floats (one 32-byte sector) in one request: SASS LDG.E.256
-__device__ __forceinline__ void ldg256(float (&d)[8], const float* src) {
-  asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3]), "=f"(d[4]), "=f"(d[5]), "=f"(d[6]), "=f"(d[7])
-               : "l"(src));
-}
-// fp16x2 {lo = a0, hi = a1}, round-to-nearest, |x| > 65504 saturates instead of becoming inf: SASS F2FP.SATFINITE.F16.F32.PACK_AB
-__device__ __forceinline__ uint32_t cvt_f16x2_sat(float a0, float a1) {
-  uint32_t h;
-  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(h) : "f"(a1), "f"(a0));
-  return h;
-}
-
-// e4m3x2 {byte 0 = a0, byte 1 = a1}, round-to-nearest, saturating at +-448
-__device__ __forceinline__ uint32_t cvt_e4m3x2_sat(float a0, float a1) {
-  unsigned short h;
-  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(h) : "f"(a1), "f"(a0));
-  return (uint32_t)h;
-}
-
-// UMMA shared-memory descriptor, no-swizzle K-major: core matrix = 8 rows x 16 B stored contiguously (128 B);
-// LBO = byte distance between the two 16-byte K-chunks of one K=16 (FP16) MMA, SBO = byte distance between 8-row groups.
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3fff);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3fff) << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3fff) << 32;
-  d |= (uint64_t)1 << 46;   // descriptor version (Blackwell)
-  return d;                 // layout_type = SWIZZLE_NONE (0), base_offset = 0
-}
-
-// kind::f16 with FP16 operands (a_format = b_format = 0), fp32 accumulate, A and B K-major, M = 128
-__device__ __forceinline__ uint32_t umma_idesc_f16(int n) {
-  return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
-
-__device__ __forceinline__ long long gtime() {
-  long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
 // debug timeline: slot 0/1 transform first-load-issue / last-store of the item, 2/3 MMA start / all issued, 4/5 epilogue start / end
 // (compiled in only with -DFS2_TC_TRACE: the checks cost ~8 % of the transform warps' instructions)
 #ifdef FS2_TC_TRACE
@@ -209,14 +90,6 @@ __device__ __forceinline__ long long gtime() {
 #else
 #define TC_STAMP(il, slot) do { } while (0)
 #endif
-
-// mbarrier ring cursor without runtime div/mod (an integer division per tap was on the MMA issuer's critical path)
-struct Ring {
-  uint32_t idx = 0, phase = 0;
-  __device__ __forceinline__ void advance(uint32_t n) {
-    if (++idx == n) { idx = 0; phase ^= 1u; }
-  }
-};
 
 struct Item { int nblk, b, t0; };
 __device__ __forceinline__ Item decode_item(const TcP& p, int item) {
@@ -364,13 +237,6 @@ __device__ __forceinline__ void tc_epilogue_dispatch(const TcP& p, uint32_t tmem
   }
 }
 
-// Operand scales of the f16 + f8 split (TcP::f8): activation lo * 2^12 and hi (unscaled) are rounded to E4M3; the packer stores
-// weight hi * 2^-12 and lo (unscaled) in E4M3 (packing.pack_conv_tc), so both correction products carry the main term's scale.
-// |x| <= 448 stays inside E4M3; beyond that the correction of that element saturates (the result degrades towards single-pass
-// fp16 accuracy for it, never to garbage).
-constexpr float TC_F8_LO_SCALE = 4096.f;
-constexpr float TC_F8_HI_SCALE = 1.f;
-
 // One K-block of one transform thread: input activation, operand split, stores into the slab planes.
 //   F8 = false: plane 0 = fp16 hi, plane 1 = fp16 lo, both [16-byte K-chunk of 8 channels][row][8 halfs].
 //   F8 = true : plane 0 = fp16 hi as above; plane 1 = E4M3 [chunk 0: lo * 2^12 of the 16 channels | chunk 1: hi of the 16 channels][row][16 bytes]
@@ -378,33 +244,20 @@ constexpr float TC_F8_HI_SCALE = 1.f;
 template <bool LRELU, bool F8, int LD>
 __device__ __forceinline__ void tc_convert_store(const float (&src)[LD][8], const int (&rowu)[LD], const int (&offu)[LD], const int (&off8)[LD],
                                                  unsigned char* hi, unsigned char* lo, uint32_t chunk_bytes, float in_slope) {
+  const auto act = [in_slope](float v) { return LRELU ? fmaxf(v, v * in_slope) : v; };   // leaky_relu for 0 <= slope <= 1
 #pragma unroll
   for (int u = 0; u < LD; u++) {
     if (rowu[u] < 0) continue;
     uint32_t hw[4], lw[4];
-#pragma unroll
-    for (int j = 0; j < 4; j++) {
-      float a0 = src[u][2 * j], a1 = src[u][2 * j + 1];
-      if (LRELU) {
-        a0 = fmaxf(a0, a0 * in_slope);                 // leaky_relu for 0 <= slope <= 1
-        a1 = fmaxf(a1, a1 * in_slope);
-      }
-      hw[j] = cvt_f16x2_sat(a0, a1);
-      const float2 hf = __half22float2(*reinterpret_cast<const __half2*>(&hw[j]));
-      if (F8) {
-        const uint32_t l8 = cvt_e4m3x2_sat((a0 - hf.x) * TC_F8_LO_SCALE, (a1 - hf.y) * TC_F8_LO_SCALE);   // a - hi is exact in fp32
-        const uint32_t h8 = cvt_e4m3x2_sat(hf.x, hf.y);                                                    // TC_F8_HI_SCALE == 1
-        if (j & 1) { lw[j >> 1] |= l8 << 16; lw[2 + (j >> 1)] |= h8 << 16; }
-        else { lw[j >> 1] = l8; lw[2 + (j >> 1)] = h8; }
-      } else {
-        lw[j] = cvt_f16x2_sat(a0 - hf.x, a1 - hf.y);
-      }
-    }
-    *reinterpret_cast<uint4*>(hi + offu[u]) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
     if (F8) {
-      *reinterpret_cast<uint2*>(lo + off8[u]) = make_uint2(lw[0], lw[1]);                 // E4M3 lo of these 8 channels
-      *reinterpret_cast<uint2*>(lo + off8[u] + chunk_bytes) = make_uint2(lw[2], lw[3]);   // E4M3 hi of these 8 channels
+      uint32_t l8[2], h8[2];
+      split_f16_e4m3(src[u], hw, l8, h8, act);
+      *reinterpret_cast<uint4*>(hi + offu[u]) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
+      *reinterpret_cast<uint2*>(lo + off8[u]) = make_uint2(l8[0], l8[1]);                  // E4M3 lo of these 8 channels
+      *reinterpret_cast<uint2*>(lo + off8[u] + chunk_bytes) = make_uint2(h8[0], h8[1]);    // E4M3 hi of these 8 channels
     } else {
+      split_f16(src[u], hw, lw, act);
+      *reinterpret_cast<uint4*>(hi + offu[u]) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
       *reinterpret_cast<uint4*>(lo + offu[u]) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
     }
   }
@@ -435,12 +288,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv_tc_kernel(const TcP p) {
     for (int i = 0; i < TC_SA_MAX; i++) { mbar_init(&fullA[i], TC_TW); mbar_init(&emptyA[i], 1); }
     for (int i = 0; i < TC_SB_MAX; i++) { mbar_init(&fullB[i], 1); mbar_init(&emptyB[i], 1); }
     for (int i = 0; i < 2; i++) { mbar_init(&accFull[i], 1); mbar_init(&accEmpty[i], 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, p.tmem_cols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -489,8 +339,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv_tc_kernel(const TcP p) {
     // elected lane issues the MMAs and the commits.  Per weight stage the 6*MT MMAs are fully unrolled and every operand is
     // a precomputed base plus a constant: the issue cost per MMA must stay well below the 16..64 cycles an MMA occupies
     // the tensor pipe (a generic address computation per MMA was measured to be the bottleneck).
-    uint32_t leader;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(leader));
+    const uint32_t leader = elect_one();
     const uint32_t idesc = umma_idesc_f16(NB);
     const uint64_t a_const = umma_desc(0, (uint32_t)R * 16, 128), b_const = umma_desc(0, (uint32_t)NB * 16, 128);
     const uint32_t tile_cols = (uint32_t)(TG * p.acc_stride);
@@ -714,7 +563,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv_tc_kernel(const TcP p) {
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(p.tmem_cols));
+    tmem_dealloc(tmem, p.tmem_cols);
   }
 }
 

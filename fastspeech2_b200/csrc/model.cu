@@ -32,8 +32,15 @@ DevState* dev_state(int* err) {
   }
   return d;
 }
-DevOnce::DevOnce() { g_dev_mutex.lock(); }
-DevOnce::~DevOnce() { g_dev_mutex.unlock(); }
+int setup_once(std::atomic<bool>& done, cudaError_t (*fn)()) {
+  if (done.load(std::memory_order_acquire)) return FS2_OK;
+  std::lock_guard<std::mutex> lock(g_dev_mutex);
+  if (done.load(std::memory_order_relaxed)) return FS2_OK;
+  const cudaError_t e = fn();
+  if (e != cudaSuccess) return FS2_ERR_CUDA - (int)e;
+  done.store(true, std::memory_order_release);
+  return FS2_OK;
+}
 
 // ------------------------------------------------------------------ per-launch profiling (off unless armed; state is per host thread)
 thread_local bool g_prof_on = false;

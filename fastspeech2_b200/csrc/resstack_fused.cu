@@ -10,7 +10,7 @@
 //     the full slab, garbage from the slab edges grows inward by one conv radius per layer and by construction stays inside the
 //     H-row halo (halo recompute); rows outside the utterance [0, N) are forced to zero after every layer (Conv1d zero padding).
 //   * activations live in shared memory ALREADY in tensor-core operand form: per 16-channel K-block an fp16 "hi" plane and an
-//     E4M3 plane [lo * 2^12 | hi * 2] (the two-MMA operand split of conv_tc_kernel.cuh, FS2_TC_VARIANT_F8), UMMA no-swizzle
+//     E4M3 plane [lo * 2^12 | hi] (the two-MMA operand split of conv_tc_kernel.cuh, FS2_TC_VARIANT_F8), UMMA no-swizzle
 //     K-major [16-byte K-chunk][row][16 B], so a conv tap is the same slab with the descriptor start advanced by tap*dilation
 //     rows.  Two slabs: XA = lrelu(x) (conv1's operand), XT = lrelu(conv1 output) (conv2's operand).
 //   * the residual stream x stays in TENSOR MEMORY in fp32 (MT*C columns) next to the MT accumulators (MT*C columns):
@@ -30,7 +30,8 @@
 
 #include <type_traits>
 
-#include "conv_tc_kernel.cuh"
+#include "common.cuh"
+#include "tc_format.cuh"
 
 namespace fs2 {
 
@@ -51,68 +52,17 @@ struct RsP {
   int accumulate;                // the first kernel size reduce-adds into y too
 };
 
-// ------------------------------------------------------------------ TMA (tensor-map) wrappers
-__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* tm, int c0, int n0, int b, uint64_t* bar) {
-  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(
-                   smem_u32(dst)),
-               "l"(reinterpret_cast<uint64_t>(tm)), "r"(c0), "r"(n0), "r"(b), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* tm, int c0, int n0, int b, const void* src) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.tile.bulk_group [%0, {%1, %2, %3}], [%4];" ::"l"(reinterpret_cast<uint64_t>(tm)),
-               "r"(c0), "r"(n0), "r"(b), "r"(smem_u32(src))
-               : "memory");
-}
-__device__ __forceinline__ void tma_reduce_add_3d(const CUtensorMap* tm, int c0, int n0, int b, const void* src) {
-  asm volatile("cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group [%0, {%1, %2, %3}], [%4];" ::"l"(
-                   reinterpret_cast<uint64_t>(tm)),
-               "r"(c0), "r"(n0), "r"(b), "r"(smem_u32(src))
-               : "memory");
-}
-__device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_reads() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-template <int NTHREADS>
-__device__ __forceinline__ void row_warps_sync() { asm volatile("bar.sync 1, %0;" ::"n"(NTHREADS) : "memory"); }   // the row warps only
-// byte offset of 16-byte chunk c of row r inside a [rows][128 B] box written / read by TMA with CU_TENSOR_MAP_SWIZZLE_128B
-__device__ __forceinline__ uint32_t sw128(int r, int c) { return (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)); }
-
-__device__ __forceinline__ void tc_st16(uint32_t taddr, const uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
-      "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]),
-      "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-      : "memory");
-}
-__device__ __forceinline__ void tc_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tc_ld16_nowait(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
 // 16 channels of one slab row -> operand planes of K-block kb (fp16 hi: two 16-byte chunks; E4M3: [lo*2^12 | hi*2]).
 // `a` already carries the activation and the out-of-utterance zeroing.
 __device__ __forceinline__ void rs_store16(unsigned char* kblk, uint32_t chunk_bytes, int row, const float (&a)[16]) {
-  uint32_t hw[8], l8[4], h8[4];
-#pragma unroll
-  for (int j = 0; j < 8; j++) {
-    const float a0 = a[2 * j], a1 = a[2 * j + 1];
-    hw[j] = cvt_f16x2_sat(a0, a1);
-    const float2 hf = __half22float2(*reinterpret_cast<const __half2*>(&hw[j]));
-    const uint32_t l = cvt_e4m3x2_sat((a0 - hf.x) * TC_F8_LO_SCALE, (a1 - hf.y) * TC_F8_LO_SCALE);
-    const uint32_t h = cvt_e4m3x2_sat(hf.x, hf.y);          // TC_F8_HI_SCALE == 1
-    if (j & 1) { l8[j >> 1] |= l << 16; h8[j >> 1] |= h << 16; }
-    else { l8[j >> 1] = l; h8[j >> 1] = h; }
-  }
+  uint32_t hw[2][4], l8[2][2], h8[2][2];
+  split_f16_e4m3(a, hw[0], l8[0], h8[0]);
+  split_f16_e4m3(a + 8, hw[1], l8[1], h8[1]);
   unsigned char* p0 = kblk + (size_t)row * 16;
-  *reinterpret_cast<uint4*>(p0) = make_uint4(hw[0], hw[1], hw[2], hw[3]);                       // plane 0, chunk 0: channels 0-7
-  *reinterpret_cast<uint4*>(p0 + chunk_bytes) = make_uint4(hw[4], hw[5], hw[6], hw[7]);         // plane 0, chunk 1: channels 8-15
-  *reinterpret_cast<uint4*>(p0 + 2 * chunk_bytes) = make_uint4(l8[0], l8[1], l8[2], l8[3]);     // plane 1, chunk 0: E4M3 lo
-  *reinterpret_cast<uint4*>(p0 + 3 * chunk_bytes) = make_uint4(h8[0], h8[1], h8[2], h8[3]);     // plane 1, chunk 1: E4M3 hi
+  *reinterpret_cast<uint4*>(p0) = make_uint4(hw[0][0], hw[0][1], hw[0][2], hw[0][3]);                   // plane 0, chunk 0: channels 0-7
+  *reinterpret_cast<uint4*>(p0 + chunk_bytes) = make_uint4(hw[1][0], hw[1][1], hw[1][2], hw[1][3]);     // plane 0, chunk 1: channels 8-15
+  *reinterpret_cast<uint4*>(p0 + 2 * chunk_bytes) = make_uint4(l8[0][0], l8[0][1], l8[1][0], l8[1][1]); // plane 1, chunk 0: E4M3 lo
+  *reinterpret_cast<uint4*>(p0 + 3 * chunk_bytes) = make_uint4(h8[0][0], h8[0][1], h8[1][0], h8[1][1]); // plane 1, chunk 1: E4M3 hi
 }
 
 __device__ __forceinline__ float rs_lrelu(float v) { return fmaxf(v, 0.1f * v); }   // LRELU_SLOPE = 0.1 (hifigan/models.py:7)
@@ -162,14 +112,11 @@ __global__ void __launch_bounds__(64 + 8 * C, 1) resstack_kernel(const __grid_co
     for (int i = 0; i < RS_SB_MAX; i++) { mbar_init(&fullB[i], 1); mbar_init(&emptyB[i], 1); }
     for (int i = 0; i < 4; i++) { mbar_init(&accFull[i], 1); mbar_init(&rowsReady[i], NRW); }
     mbar_init(xLoaded, 1); mbar_init(xaFree, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmx)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmy)) : "memory");
+    mbar_init_fence();
+    tma_prefetch_map(&tmx);
+    tma_prefetch_map(&tmy);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
   fence_proxy_async();
   tc_fence_before();
   __syncthreads();
@@ -202,8 +149,7 @@ __global__ void __launch_bounds__(64 + 8 * C, 1) resstack_kernel(const __grid_co
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    uint32_t leader;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(leader));
+    const uint32_t leader = elect_one();
     const uint32_t idesc = umma_idesc_f16(C);
     const uint64_t a_const = umma_desc(0, CHUNK, 128), b_const = umma_desc(0, (uint32_t)C * 16, 128);
     const uint32_t xa16 = smem_u32(xa) >> 4, xt16 = smem_u32(xt) >> 4;
@@ -431,7 +377,7 @@ __global__ void __launch_bounds__(64 + 8 * C, 1) resstack_kernel(const __grid_co
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS));
+    tmem_dealloc(tmem, TMEM_COLS);
   }
 }
 
@@ -533,17 +479,13 @@ int resstack(const fs2_resstack_args* a, cudaStream_t s) {
   if (!dv) return derr;
   int plan[12];
   FS2_TRY(resstack_plan(a, dv->num_sms.load(std::memory_order_relaxed), plan));
-  if (!dv->fused_ready.load(std::memory_order_acquire)) {
-    DevOnce once;
-    if (!dv->fused_ready.load(std::memory_order_relaxed)) {
-      const int mx = 227 * 1024;
-      cudaError_t e = cudaFuncSetAttribute(resstack_kernel<32, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
-      if (e == cudaSuccess) e = cudaFuncSetAttribute(resstack_kernel<64, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
-      if (e == cudaSuccess) e = cudaFuncSetAttribute(resstack_kernel<32, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
-      if (e != cudaSuccess) return FS2_ERR_CUDA - (int)e;
-      dv->fused_ready.store(true, std::memory_order_release);
-    }
-  }
+  FS2_TRY(setup_once(dv->fused_ready, [] {
+    const int mx = 227 * 1024;
+    cudaError_t e = cudaFuncSetAttribute(resstack_kernel<32, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(resstack_kernel<64, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(resstack_kernel<32, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+    return e;
+  }));
   RsP p{};
   p.B = a->B; p.N = a->N;
   p.n_kernels = a->n_kernels; p.n_dil = a->n_dil;
